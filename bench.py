@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the KnightVision B200 hot path (contract: see the task / DESIGN.md §measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload mcts|perft] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload mcts|perft] [--impl ours|reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1; RANK/LOCAL_RANK/WORLD_SIZE from the env).  Rank 0 prints ONE JSON line.
 Workloads:
@@ -12,6 +12,8 @@ Workloads:
   learn  BASELINE.json configs[4]: whole loop iterations, self-play feeding training (bench_learn.py).
 `--impl reference` times the CPU implementation of the same path (the oracle port, all host cores) on a bounded
 sample of the same workload.
+`--dump-outputs DIR` (mcts) writes what the timed window's last move left a caller as DIR/<name>.npy, so that two builds
+can be compared output for output on identical (seeded) inputs; see bench_mcts.collect_outputs (rank 0's games only).
 """
 from __future__ import annotations
 
@@ -404,9 +406,22 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=None, choices=["mcts", "perft", "train", "learn"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (mcts workload)")
     args, _ = ap.parse_known_args()
     if args.workload is None:
         args.workload = "mcts" if os.path.exists(os.path.join(ROOT, "bench_mcts.py")) else "perft"
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "ours" or args.workload != "mcts":
+            ap.error("--dump-outputs is implemented for the mcts workload of --impl ours")
+        try:                        # a directory that cannot be written fails here, before any GPU work
+            os.makedirs(args.dump_outputs, exist_ok=True)
+        except OSError as e:
+            ap.error(f"--dump-outputs: {e}")
+        if not os.access(args.dump_outputs, os.W_OK | os.X_OK):
+            ap.error(f"--dump-outputs: {args.dump_outputs} is not writable")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -190,6 +190,54 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_RECORDS = 8192     # records --dump-outputs writes at most: their planes are 25 MB
+
+
+def dump_games(n_games, moves):
+    """Games --dump-outputs writes after `moves` moves since the reset: all of them, or a fixed sample (seed 0) of
+    DUMP_RECORDS // moves games, ascending.  A game records at most one position per move, so the sample holds at most
+    DUMP_RECORDS records; it depends on the bench's arguments only, not on how the games went."""
+    k = max(1, min(n_games, DUMP_RECORDS // max(moves, 1)))
+    if k == n_games:
+        return np.arange(n_games)
+    return np.sort(np.random.default_rng(0).choice(n_games, k, replace=False))
+
+
+def collect_outputs(eng, moves):
+    """bench.py --dump-outputs: host copies of what a caller of the self-play path holds after the last move, for the
+    games of dump_games (this rank's games: with several GPUs, rank 0's shard).
+      games          float64 [S]          the sampled games (index within this rank's games)
+      roots          float32 [S, 64]      their current positions: the 16 int64 words as 16-bit limbs (exact)
+      counters       float64 [6]          over all games: done, plies played, edge-pool overflows, white wins, black
+                                          wins, draws
+      record_planes  float32 [R, 12, 8, 8] \\
+      record_move    float64 [R]            every record of the sampled games in the reference's format (planes, move
+      record_reward  float32 [R]            index, reward; SelfPlay.records), in game order, and the game it belongs to
+      record_game    float64 [R]          /
+    Under 28 MB in all (at most DUMP_RECORDS records)."""
+    import torch
+    games = dump_games(eng.mcts_games, moves)
+    lines, move, reward, game = eng.mcts_records()
+    sel = torch.nonzero(torch.isin(game, torch.from_numpy(games).to(game.device, game.dtype)))[:, 0]
+    st = eng.mcts_status()
+    return {
+        "games": games.astype(np.float64),
+        "roots": eng.mcts_roots().cpu().numpy()[games].view(np.uint16).astype(np.float32),
+        "counters": np.array([st[k] for k in ("done", "plies", "overflow", "white_wins", "black_wins", "draws")],
+                             np.float64),
+        "record_planes": eng.encode(lines[sel].contiguous()).cpu().numpy(),
+        "record_move": move[sel].cpu().numpy().astype(np.float64),
+        "record_reward": reward[sel].cpu().numpy(),
+        "record_game": game[sel].cpu().numpy().astype(np.float64),
+    }
+
+
+def save_outputs(out_dir, outputs):
+    """collect_outputs' arrays as out_dir/<name>.npy."""
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _gather_list(x, world, dev):
     """all_gather of one float per rank -> python list (rank order)."""
     import torch
@@ -278,6 +326,8 @@ def run(args, rank, world, local_rank):
     snapshot_h = eng.mcts_roots().cpu().pin_memory()      # positions at the start of the timed region (for B and C)
     clocks.start()
     dev_ms, st0, st1, prof, launches = timed_moves(args.steps, profile=True)
+    # host copies now (phase B resets the games); the files are written once the clock sampler has stopped
+    outputs = collect_outputs(eng, warm + args.steps) if args.dump_outputs and rank == 0 else None
     # simulations actually run, from the device's ply counter: a game plays a ply only after its SIMS simulations, and a
     # game that ended inside the window stops contributing
     positions = st1["plies"] - st0["plies"]
@@ -336,6 +386,8 @@ def run(args, rank, world, local_rank):
     tuples_ms = (time.perf_counter() - tt) * 1e3
     e2e_s = time.perf_counter() - t0
     clk = clocks.stop()
+    if outputs is not None:
+        save_outputs(args.dump_outputs, outputs)
     e2e_positions = e1["plies"] - e0["plies"]
     gather_bytes = int(lines_r.shape[0]) * (16 * 8 + 4 + 4 + 8)
 

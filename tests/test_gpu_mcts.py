@@ -117,6 +117,43 @@ def test_dropin_self_play_record_format(eng, monkeypatch):
         SP.self_play(None, 1, torch.device("cuda:0"), model_path="/nonexistent/model.pth")
 
 
+def test_bench_dump_outputs(eng, tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float arrays that hold the roots exactly and the records as SelfPlay.records returns them;
+    beyond DUMP_RECORDS records, every record of a fixed sample of games, the same on every call."""
+    import bench_mcts as B
+    from knightvision_b200.selfplay import records_to_tuples
+    G, moves = 40, 5
+    eng.mcts_create(G, 16, max_plies=30, temp_plies=4, seed=11, eval_mode=0)
+    eng.mcts_reset(None, game_id_base=0)
+    for _ in range(moves):
+        eng.mcts_run_move()
+    B.save_outputs(str(tmp_path), B.collect_outputs(eng, moves))
+    got = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert sorted(got) == ["counters", "games", "record_game", "record_move", "record_planes", "record_reward", "roots"]
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert got["games"].tolist() == list(range(G))
+    roots = got["roots"].astype(np.uint16).view(np.int64)
+    assert np.array_equal(roots, eng.mcts_roots().cpu().numpy())
+    st = eng.mcts_status()
+    assert got["counters"].tolist() == [st["done"], st["plies"], st["overflow"], st["white_wins"], st["black_wins"], st["draws"]]
+    lines, move, reward, game = eng.mcts_records()
+    recs = records_to_tuples(eng, lines, move, reward)
+    assert len(recs) == st["plies"] > 64
+    assert np.array_equal(got["record_planes"], np.stack([r[0] for r in recs]))
+    assert got["record_move"].tolist() == [r[1] for r in recs] and got["record_reward"].tolist() == [r[2] for r in recs]
+    assert np.array_equal(got["record_game"], game.cpu().numpy())
+
+    monkeypatch.setattr(B, "DUMP_RECORDS", 64)
+    a, b = B.collect_outputs(eng, moves), B.collect_outputs(eng, moves)
+    games = B.dump_games(G, moves)
+    assert len(games) == 64 // moves and np.array_equal(a["games"], games)
+    keep = np.isin(got["record_game"], games)
+    assert len(a["record_game"]) <= 64 and set(a["record_game"].tolist()) == set(games.tolist())
+    for name in ("record_planes", "record_move", "record_reward", "record_game"):
+        assert np.array_equal(a[name], got[name][keep]) and np.array_equal(a[name], b[name]), name
+    assert np.array_equal(a["roots"], got["roots"][games])
+
+
 def test_full_size_wave_4096_games(eng):
     """BASELINE config 3 size: 4 096 concurrent games; size-independent invariants after 12 waves."""
     from knightvision_b200.model import ChessNet
