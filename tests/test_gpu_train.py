@@ -123,10 +123,14 @@ def test_training_step_native_vs_cudnn(eng, monkeypatch):
     assert d < 5e-3, d
 
 
-@pytest.mark.parametrize("rows_boards,C,with_res", [(3, 256, False), (77, 512, True), (512, 256, True)])
-def test_bn_relu_fwd_bwd_match_torch_fp32(eng, rows_boards, C, with_res):
+@pytest.mark.parametrize("rows_boards,C,with_res,relu", [
+    pytest.param(3, 256, False, True, id="3-256-False"), pytest.param(77, 512, True, True, id="77-512-True"),
+    pytest.param(512, 256, True, True, id="512-256-True"), pytest.param(5, 64, True, True, id="5-64-True"),
+    pytest.param(33, 128, False, True, id="33-128-False"), pytest.param(9, 1024, True, True, id="9-1024-True"),
+    pytest.param(40, 256, True, False, id="40-256-True-norelu"), pytest.param(7, 1024, False, False, id="7-1024-False-norelu")])
+def test_bn_relu_fwd_bwd_match_torch_fp32(eng, rows_boards, C, with_res, relu):
     """Fused train-mode BatchNorm + ReLU (+ residual) against torch fp32 on the same bf16 inputs: outputs, input / skip /
-    affine gradients, saved and running statistics."""
+    affine gradients, saved and running statistics, at every supported C and with the ReLU on or off."""
     n = rows_boards
     g = torch.Generator(device="cuda").manual_seed(C + n)
     z = (torch.randn(n, 8, 8, C, device="cuda", generator=g) * 1.7 + 0.3).to(torch.bfloat16)
@@ -135,15 +139,17 @@ def test_bn_relu_fwd_bwd_match_torch_fp32(eng, rows_boards, C, with_res):
     gamma = (torch.rand(C, device="cuda", generator=g) + 0.5)
     beta = torch.randn(C, device="cuda", generator=g) * 0.2
     rm, rv = torch.zeros(C, device="cuda"), torch.ones(C, device="cuda")
-    y, mean, rstd = eng.bn_relu_fwd(z, gamma, beta, rm, rv, 0.1, 1e-5, residual=res, relu=True)
-    dz, dres, dgamma, dbeta = eng.bn_relu_bwd(dy, y, z, gamma, mean, rstd, relu=True, want_dres=with_res)
+    y, mean, rstd = eng.bn_relu_fwd(z, gamma, beta, rm, rv, 0.1, 1e-5, residual=res, relu=relu)
+    dz, dres, dgamma, dbeta = eng.bn_relu_bwd(dy, y, z, gamma, mean, rstd, relu=relu, want_dres=with_res)
     # torch fp32 reference
     zf = z.float().permute(0, 3, 1, 2).clone().requires_grad_()
     gf, bf = gamma.clone().requires_grad_(), beta.clone().requires_grad_()
     rf = res.float().permute(0, 3, 1, 2).clone().requires_grad_() if with_res else None
     rm2, rv2 = torch.zeros(C, device="cuda"), torch.ones(C, device="cuda")
     pre = F.batch_norm(zf, rm2, rv2, gf, bf, True, 0.1, 1e-5)
-    out = F.relu(pre + rf if with_res else pre)
+    out = pre + rf if with_res else pre
+    if relu:
+        out = F.relu(out)
     # the kernel masks with its own bf16 output; use the same mask for the reference gradient where out is within rounding of 0
     out.backward(dy.float().permute(0, 3, 1, 2))
     assert _rel(y.permute(0, 3, 1, 2), out.detach()) < 6e-3
