@@ -836,6 +836,17 @@ static int choose_move(const kvo_mcts_cfg *cfg, const oedge *e, int n, uint64_t 
     return pick;
 }
 
+/* Optional copy of the whole tree at the end of a search (kvo_mcts_search_tree); NULL members are skipped. */
+typedef struct {
+    uint64_t *node_line;   /* [sims + 1][16] the node's line as stored after move generation (the evaluated position) */
+    int32_t *node_i32;     /* [sims + 1][4]  terminal flag, first edge (-1 none), edge count, visits N */
+    float *node_val;       /* [sims + 1]     terminal value or the evaluator's value, from the node's side to move */
+    uint16_t *edge_mv;     /* [edge_cap]     move word */
+    int32_t *edge_child;   /* [edge_cap]     child node, -1 unexpanded */
+    float *edge_P, *edge_W;
+    uint32_t *edge_N;
+} tree_out_t;
+
 /* Runs one search of cfg->sims simulations from `root`; returns the chosen move word (0xFFFF if the root has no
  * move).  Outputs: root move list, visit counts, W (bit patterns), number of nodes/edges created.
  *
@@ -848,7 +859,7 @@ static int choose_move(const kvo_mcts_cfg *cfg, const oedge *e, int n, uint64_t 
  * computed). */
 static int mcts_search(const kvo_mcts_cfg *cfg, const kvo_state *root, uint64_t game_id, int ply, const replay_t *rep,
                        uint16_t *root_moves, uint32_t *root_N, float *root_W, float *root_P, int *n_root,
-                       int *out_nodes, int *out_edges, int *overflow, float *root_vwhite) {
+                       int *out_nodes, int *out_edges, int *overflow, float *root_vwhite, const tree_out_t *tout) {
     const int S = cfg->sims;
     const int K = cfg->inflight > 1 ? cfg->inflight : 1;
     const size_t PL = (size_t)S + 2;   /* path stride */
@@ -998,6 +1009,26 @@ static int mcts_search(const kvo_mcts_cfg *cfg, const kvo_state *root, uint64_t 
     }
     *out_nodes = n_nodes;
     *out_edges = n_edges;
+    if (tout) {
+        for (int i = 0; i < n_nodes; i++) {
+            if (tout->node_line) kvo_pack(&nodes[i].st, tout->node_line + (size_t)i * 16);
+            if (tout->node_i32) {
+                int32_t *o = tout->node_i32 + (size_t)i * 4;
+                o[0] = nodes[i].term;
+                o[1] = nodes[i].first_edge;
+                o[2] = nodes[i].n_edges;
+                o[3] = (int32_t)nodes[i].N;
+            }
+            if (tout->node_val) tout->node_val[i] = nodes[i].val;
+        }
+        for (int i = 0; i < n_edges; i++) {
+            if (tout->edge_mv) tout->edge_mv[i] = edges[i].mv;
+            if (tout->edge_child) tout->edge_child[i] = edges[i].child;
+            if (tout->edge_P) tout->edge_P[i] = edges[i].P;
+            if (tout->edge_W) tout->edge_W[i] = edges[i].W;
+            if (tout->edge_N) tout->edge_N[i] = edges[i].N;
+        }
+    }
     free(nodes);
     free(edges);
     free(path_e);
@@ -1016,12 +1047,46 @@ KVO_API int kvo_mcts_search(const kvo_mcts_cfg *cfg, const uint64_t *line, uint6
     replay_t rep = { rep_node_val, rep_node_first, rep_edge_P };
     int n_root, nn, ne, ov;
     int mv = mcts_search(cfg, &s, game_id, ply, rep_node_val ? &rep : NULL, root_moves, root_N, root_W, root_P, &n_root,
-                         &nn, &ne, &ov, NULL);
+                         &nn, &ne, &ov, NULL, NULL);
     info4[0] = n_root;
     info4[1] = nn;
     info4[2] = ne;
     info4[3] = ov;
     return mv;
+}
+
+/* kvo_mcts_search, and a copy of the tree it built (hash or replay mode): per node node_line [sims + 1][16],
+ * node_i32 [sims + 1][4] = (terminal, first edge, edge count, N), node_val [sims + 1]; per edge [cfg->edge_cap] the
+ * move word, child node, prior P, value sum W and visits N.  Nodes and edges are numbered in creation order, as on the
+ * device.  Every output pointer may be NULL. */
+KVO_API int kvo_mcts_search_tree(const kvo_mcts_cfg *cfg, const uint64_t *line, uint64_t game_id, int ply,
+                                 const float *rep_node_val, const int32_t *rep_node_first, const float *rep_edge_P,
+                                 uint16_t *root_moves, uint32_t *root_N, float *root_W, float *root_P, int32_t *info4,
+                                 uint64_t *node_line, int32_t *node_i32, float *node_val, uint16_t *edge_mv,
+                                 int32_t *edge_child, float *edge_P, float *edge_W, uint32_t *edge_N) {
+    kvo_state s;
+    kvo_unpack(line, &s);
+    replay_t rep = { rep_node_val, rep_node_first, rep_edge_P };
+    const tree_out_t tout = { node_line, node_i32, node_val, edge_mv, edge_child, edge_P, edge_W, edge_N };
+    int n_root, nn, ne, ov;
+    int mv = mcts_search(cfg, &s, game_id, ply, rep_node_val ? &rep : NULL, root_moves, root_N, root_W, root_P, &n_root,
+                         &nn, &ne, &ov, NULL, &tout);
+    info4[0] = n_root;
+    info4[1] = nn;
+    info4[2] = ne;
+    info4[3] = ov;
+    return mv;
+}
+
+/* test helper: the root noise eta[k] of priors_from_logits for a root with n legal moves (Gamma variates keyed by
+ * ply * 256 + k, divided by their sequential sum) */
+KVO_API void kvo_root_eta(float alpha, uint64_t seed, uint64_t game_id, int ply, int n, float *out) {
+    float gs = 0.0f;
+    for (int k = 0; k < n; k++) {
+        out[k] = kvd_gamma_small(alpha, seed, game_id, (uint64_t)ply * 256 + (uint64_t)k);
+        gs = gs + out[k];
+    }
+    for (int k = 0; k < n; k++) out[k] = out[k] / gs;
 }
 
 /* test helper: the Gamma(alpha) variates the reference-rule root noise draws for every policy index */
@@ -1071,7 +1136,7 @@ KVO_API int kvo_selfplay_game2(const kvo_mcts_cfg *cfg, const uint64_t *start_li
         if (ply == 0 && (f & RF_ONLY_KINGS)) break;      /* a start position without pieces: nothing to search */
         int n_root, nn, ne, ov;
         float vroot = 0.0f;
-        int mv = mcts_search(cfg, &s, game_id, ply, NULL, rm, rn, rw, rp, &n_root, &nn, &ne, &ov, &vroot);
+        int mv = mcts_search(cfg, &s, game_id, ply, NULL, rm, rn, rw, rp, &n_root, &nn, &ne, &ov, &vroot, NULL);
         if (ply < script_n) {
             if (script_vals && script_vals[ply] == script_vals[ply]) vroot = script_vals[ply];
             if (script_moves && script_moves[ply] != 0xFFFF) {

@@ -112,9 +112,13 @@ def mcts_cfg(sims, edges_per_node=64, temp_plies=0, max_plies=1 << 20, c_puct=1.
                    inflight, seed, resign_thr, resign_min_plies, int(sims == 1) if root_mix < 0 else root_mix, 0)
 
 
-def mcts_search(cfg, line, game_id=0, ply=0, replay=None):
+def mcts_search(cfg, line, game_id=0, ply=0, replay=None, nodes=False):
     """One search.  replay = (node_val f32[], node_first i32[], edge_P f32[]) dumps of the device tree, or None for
-    the hash evaluator.  Returns dict(move, moves, N, W, P, nodes, edges, overflow)."""
+    the hash evaluator.  Returns dict(move, moves, N, W, P, nodes, edges, overflow).
+    nodes=True adds the whole tree, numbered in creation order as on the device: node_line u64 [nodes,16] (the line as
+    stored after move generation, i.e. the position the evaluator sees), node_term, node_first (-1 none), node_n
+    (edge count), node_N, node_val (terminal or evaluator value, side to move's view); edge_mv, edge_child (-1
+    unexpanded), edge_P, edge_W, edge_N [edges]."""
     line = np.ascontiguousarray(line, dtype=np.uint64)
     moves = np.zeros(256, np.uint16); N = np.zeros(256, np.uint32); W = np.zeros(256, np.float32)
     P = np.zeros(256, np.float32); info = np.zeros(4, np.int32)
@@ -123,14 +127,38 @@ def mcts_search(cfg, line, game_id=0, ply=0, replay=None):
     else:
         rv, rf, rp = (np.ascontiguousarray(replay[0], np.float32), np.ascontiguousarray(replay[1], np.int32),
                       np.ascontiguousarray(replay[2], np.float32))
-    f = lib().kvo_mcts_search
+    args = [ctypes.byref(cfg), _p(line), ctypes.c_uint64(game_id), ctypes.c_int(ply),
+            _p(rv) if rv is not None else None, _p(rf) if rf is not None else None, _p(rp) if rp is not None else None,
+            _p(moves), _p(N), _p(W), _p(P), _p(info)]
+    if nodes:
+        nc, ec = int(cfg.sims) + 1, int(cfg.edge_cap)
+        t = dict(node_line=np.zeros((nc, 16), np.uint64), node_i32=np.zeros((nc, 4), np.int32),
+                 node_val=np.zeros(nc, np.float32), edge_mv=np.zeros(ec, np.uint16), edge_child=np.zeros(ec, np.int32),
+                 edge_P=np.zeros(ec, np.float32), edge_W=np.zeros(ec, np.float32), edge_N=np.zeros(ec, np.uint32))
+        f = lib().kvo_mcts_search_tree
+        args += [_p(a) for a in t.values()]
+    else:
+        f = lib().kvo_mcts_search
     f.restype = ctypes.c_int
-    mv = f(ctypes.byref(cfg), _p(line), ctypes.c_uint64(game_id), ctypes.c_int(ply),
-           _p(rv) if rv is not None else None, _p(rf) if rf is not None else None, _p(rp) if rp is not None else None,
-           _p(moves), _p(N), _p(W), _p(P), _p(info))
+    mv = f(*args)
     n = int(info[0])
-    return dict(move=mv, moves=moves[:n], N=N[:n], W=W[:n], P=P[:n], nodes=int(info[1]), edges=int(info[2]),
-                overflow=int(info[3]))
+    out = dict(move=mv, moves=moves[:n], N=N[:n], W=W[:n], P=P[:n], nodes=int(info[1]), edges=int(info[2]),
+               overflow=int(info[3]))
+    if nodes:
+        nn, ne = out["nodes"], out["edges"]
+        ni = t.pop("node_i32")[:nn]
+        out.update(node_term=ni[:, 0].astype(bool), node_first=ni[:, 1], node_n=ni[:, 2], node_N=ni[:, 3].astype(np.uint32))
+        out.update({k: v[:nn] if k.startswith("node") else v[:ne] for k, v in t.items()})
+    return out
+
+
+def root_eta(alpha, seed, game_id, ply, n):
+    """Root noise eta[k] (k < n legal moves) of the legal-move prior rule: Gamma(alpha) variates keyed by ply * 256 + k,
+    divided by their sequential float32 sum.  Root priors are (1 - eps) * softmax + eps * eta."""
+    out = np.zeros(max(int(n), 1), np.float32)
+    lib().kvo_root_eta(ctypes.c_float(alpha), ctypes.c_uint64(seed), ctypes.c_uint64(game_id), ctypes.c_int(ply),
+                       ctypes.c_int(int(n)), _p(out))
+    return out[:int(n)]
 
 
 def selfplay_game(cfg, start_line, game_id=0, script_moves=None, script_vals=None, return_flags=False):

@@ -125,6 +125,68 @@ def synthetic_lines(n: int, seed: int, wild: bool = True) -> np.ndarray:
     return out
 
 
+# 218 legal moves for white (R6R/3Q4/1Q4Q1/4Q3/2Q4Q/Q4Q2/pp1Q4/kBNN1KB1 w); most replies are mates or stalemates
+MANY_MOVES_BOARD = [
+    ["wR", "--", "--", "--", "--", "--", "--", "wR"],
+    ["--", "--", "--", "wQ", "--", "--", "--", "--"],
+    ["--", "wQ", "--", "--", "--", "--", "wQ", "--"],
+    ["--", "--", "--", "--", "wQ", "--", "--", "--"],
+    ["--", "--", "wQ", "--", "--", "--", "--", "wQ"],
+    ["wQ", "--", "--", "--", "--", "wQ", "--", "--"],
+    ["bp", "bp", "--", "wQ", "--", "--", "--", "--"],
+    ["bK", "wB", "wN", "wN", "--", "wK", "wB", "--"],
+]
+
+
+def search_roots(n_random: int = 20, seed: int = 61):
+    """(lines u64 [n,16], names) of search roots where evaluators go wrong: the start position; random-playout positions,
+    half with white and half with black to move; the perft golden positions (castling, e.p., promotion); a position
+    with 218 legal moves; one with an e.p. capture; a synthetic line whose move generation rewrites the board (the
+    getKingMoves restore quirk, RF_STATE_MUTATED: the position evaluated is not the line given); and three roots that
+    share the 12 bitboards (the network's whole input and the evaluation cache's key) with another root but differ in
+    side to move, castling rights or e.p. square.  (castle_w and castle_b share their bitboards too.)"""
+    gold = perft_gold()
+    lines, names = [L.start_line()], ["start"]
+    pos = random_playout_positions(n_games=8, max_plies=90, seed=seed)
+    _, counts, flags, _ = O.movegen(pos.copy())
+    ok = (counts > 0) & ((flags & L.RF_ONLY_KINGS) == 0)
+    rng = np.random.default_rng(seed)
+    for side in (1, 0):
+        cand = np.nonzero(ok & ((pos[:, 12] & np.uint64(1)) == side))[0]
+        for i in rng.choice(cand, n_random // 2, replace=False):
+            lines.append(pos[i])
+            names.append(f"playout {i} {'white' if side else 'black'} to move")
+    for k in gold:
+        if k != "startpos":
+            lines.append(np.array(gold[k]["line"], dtype=np.uint64))
+            names.append(k)
+    lines.append(L.pack_fields(MANY_MOVES_BOARD, True, wk=(7, 5), bk=(7, 0), moved=63))
+    names.append("218 moves")
+    ep = O.make_moves(np.array(gold["ep_a"]["line"], dtype=np.uint64)[None], np.array([L.move_word(1, 3, 3, 3)]))[0]
+    lines.append(ep)                                               # white can take d7-d5 e.p. at the root
+    names.append("ep_a after d7-d5")
+    syn = synthetic_lines(64, 0)
+    _, counts, flags, _ = O.movegen(syn.copy())
+    mut = np.nonzero(((flags & L.RF_STATE_MUTATED) != 0) & (counts > 0) & ((flags & L.RF_ONLY_KINGS) == 0))[0]
+    lines.append(syn[mut[0]])
+    names.append(f"synthetic {mut[0]}, board rewritten by move generation")
+    # same bitboards, other side to move (and no e.p. square); castling rights gone; e.p. square gone
+    no_ep = ~np.uint64(0x7F00)
+    flip = lines[1].copy()
+    flip[12] = ((flip[12] ^ np.uint64(1)) & no_ep) | np.uint64(L.EP_NONE << 8)
+    lines.append(flip)
+    names.append(names[1] + ", other side to move")
+    castle = np.array(gold["castle_w"]["line"], dtype=np.uint64)
+    castle[12] |= np.uint64(L.F_WK << 1)
+    lines.append(castle)
+    names.append("castle_w, king moved")
+    ep = ep.copy()
+    ep[12] = (ep[12] & no_ep) | np.uint64(L.EP_NONE << 8)
+    lines.append(ep)
+    names.append("ep_a after d7-d5 without e.p. square")
+    return np.stack(lines), names
+
+
 def oracle_attack_masks(lines: np.ndarray) -> np.ndarray:
     """squareUnderAttack for all 64 squares of every line as a bit mask (bit r*8+c), from the oracle."""
     out = np.zeros(len(lines), dtype=np.uint64)

@@ -6,6 +6,7 @@ import pytest
 import torch
 
 import helpers as H
+from netref import reference_rule_priors
 from knightvision_b200 import layout as L
 from oracle import kv_oracle as O
 
@@ -397,17 +398,6 @@ def test_evaluation_players(eng, monkeypatch):
     assert r["a_wins"] + r["b_wins"] + r["draws"] == 8 and r["games"] == 8
 
 
-def _reference_rule_priors(logits, moves, alpha, eps, seed, game_id, ply):
-    """scripts/self_play.py:150-167 in float64 (see tests/test_emu_mcts.py)."""
-    p = np.exp(logits.astype(np.float64) - logits.max())
-    p /= p.sum()
-    if eps > 0:
-        g = O.root_noise(alpha, seed, game_id, ply).astype(np.float64)
-        p = (1 - eps) * p + eps * g / g.sum()
-    w = p[[O.lib().kvo_move_index(int(m)) for m in moves]]
-    return w / w.sum()
-
-
 def test_reference_rule_mode_hash_evaluator_bit_exact(eng):
     """sims = 1: no search, the move is sampled from root priors mixed the reference's way (softmax and Dirichlet noise
     over all 4096 indices, scripts/self_play.py:150-167), resignation on.  Whole games and priors bit-exact vs the oracle."""
@@ -421,7 +411,7 @@ def test_reference_rule_mode_hash_evaluator_bit_exact(eng):
         r = O.mcts_search(cfg, L.start_line(), game_id=300 + g, ply=0)
         assert np.array_equal(got["moves"], r["moves"]) and np.array_equal(_bits(got["P"]), _bits(r["P"])), g
         lg, _ = O.hash_eval(L.start_line())
-        assert np.allclose(got["P"], _reference_rule_priors(lg, got["moves"], 0.3, 0.25, 21, 300 + g, 0), rtol=2e-5)
+        assert np.allclose(got["P"], reference_rule_priors(lg, got["moves"], 0.3, 0.25, 21, 300 + g, 0), rtol=2e-5)
     eng.mcts_finish_move()
     for _ in range(max_plies):
         eng.mcts_run_move()
@@ -459,7 +449,7 @@ def test_reference_rule_mode_network_priors(eng):
     first = {}
     for g in (0, 5, 11):
         got = eng.mcts_read_root(g)
-        want = _reference_rule_priors(lg, got["moves"], 0.3, 0.25, 8, 70 + g, 0)
+        want = reference_rule_priors(lg, got["moves"], 0.3, 0.25, 8, 70 + g, 0)
         assert np.allclose(got["P"], want, rtol=1e-3, atol=1e-6), g
         first[g] = got["P"].copy()
     # the same roots again, now served by the cache (late kernel): identical bits
@@ -476,7 +466,7 @@ def test_reference_rule_mode_network_priors(eng):
     pol, _ = net.forward_lines(torch.from_numpy(roots.view(np.int64)).to(eng.device))
     for g in (1, 7):
         got = eng.mcts_read_root(g)
-        want = _reference_rule_priors(pol[g].float().cpu().numpy(), got["moves"], 0.3, 0.25, 8, 70 + g, 2)
+        want = reference_rule_priors(pol[g].float().cpu().numpy(), got["moves"], 0.3, 0.25, 8, 70 + g, 2)
         assert np.allclose(got["P"], want, rtol=1e-3, atol=1e-6), g
     eng.mcts_enable_cache(0)
 

@@ -86,7 +86,7 @@ def test_float64_network_reference_matches_golden():
     import torch
     import helpers as H
     from oracle import kv_oracle as O
-    from test_gpu_shapes import Fp64Net, bnrand_net
+    from netref import Fp64Net, bnrand_net
     g = np.load(H.GOLDEN + "/net_wide.npz")
     for prefix, kw in (("ref_bnrand", {}), ("t20", dict(stem=256, tower=256, blocks=20, conv2=False))):
         n = 8
